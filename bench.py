@@ -46,14 +46,14 @@ def workload_spec(name, batch=0, hidden=0, n=0, steps_t=0):
             name="mlp", program="cfg3_mlp", graph="cfg3_mlp", B=B, H=H, rows="B",
             desc=f"cfg3: 2-layer tanh MLP fwd+grad (MSE), batch {B} x hidden {H}, f32 graph",
             gemm_flops=5 * 2.0 * B * H * H,            # SURVEY 8d: 5 GEMMs x 2BH^2
-            n_gemm=5, shard_inputs=(0, 1),
+            n_gemm=5, shard_inputs=(0, 1), outputs=("loss", "dW1", "db1", "dW2", "db2"),
         )
     if name == "elemwise":
         n = n or (1 << 28)
         return dict(
             name="elemwise", program="cfg2_fused", graph="cfg2_fused_elemwise", n=n, rows="n",
             desc=f"cfg2: fused Elemwise softplus(tanh(x)+y)*z on 3x{n} f32",
-            gemm_flops=0.0, n_gemm=0, shard_inputs=(0, 1, 2),
+            gemm_flops=0.0, n_gemm=0, shard_inputs=(0, 1, 2), outputs=("out",),
         )
     if name == "lstm":
         T, B, H = steps_t or 128, batch or 8192, hidden or 1024
@@ -62,6 +62,7 @@ def workload_spec(name, batch=0, hidden=0, n=0, steps_t=0):
             desc=f"cfg4: Scan LSTM cell, T={T} steps, batch {B}, hidden {H}, f32",
             gemm_flops=2.0 * T * B * H * 4 * H, n_gemm=T,      # SURVEY 8d: 8.80 TFLOP
             ideal_bytes=(T * B * 4 * H + 4 * B * H + H * 4 * H) * 4.0,  # 17.33 GB (x read once)
+            outputs=("h_T", "c_T"),
         )
     if name == "logreg":
         N, D = n or (1 << 24), hidden or 512
@@ -72,14 +73,14 @@ def workload_spec(name, batch=0, hidden=0, n=0, steps_t=0):
             graph_bytes=(2.0 * N * D + 12.0 * N) * 4,      # SURVEY 8d graph-as-optimised
             # single-pass row-region fusion (runtime/rowfuse.py): X once, y read by `1 - y` and
             # by the fused kernel, `1 - y` written and read back
-            fused_bytes=(1.0 * N * D + 4.0 * N) * 4,
+            fused_bytes=(1.0 * N * D + 4.0 * N) * 4, outputs=("cost", "grad_w", "grad_b"),
         )
     if name == "readme":
         n = n or 1000
         return dict(
             name="readme", program="cfg1_readme", graph="cfg1_readme", n=n, rows=None,
             desc=f"cfg1: README a/a + (M+a).dot(v), {n}x{n} f64",
-            gemm_flops=0.0, n_gemm=0,
+            gemm_flops=0.0, n_gemm=0, outputs=("d",),
         )
     raise SystemExit(f"unknown workload {name}")
 
@@ -495,9 +496,34 @@ def truth_check(spec, precision, outs, keep):
             "err": err, "max_err": max(err.values()), "stated_tolerance": tol, "within": max(err.values()) <= tol}
 
 
+DUMP_BUDGET = 64 * 10 ** 6  # bytes of all files together, .npy headers included
+NPY_HEADER_MAX = 4096       # np.save writes a header of at most this many bytes per file
+
+
+def dump_outputs(outs, names, d):
+    """Write the outputs of one step as ``d/<name>.npy`` (float32 / float64).  An output larger
+    than its even share of DUMP_BUDGET (after the headers) is written as the flat elements at
+    sorted positions drawn with ``np.random.default_rng(0)``, the same on every run."""
+    from aesara_b200.runtime.device import DeviceArray
+
+    outs = outs if isinstance(outs, (list, tuple)) else [outs]
+    assert len(outs) == len(names), (len(outs), names)
+    os.makedirs(d, exist_ok=True)
+    share = (DUMP_BUDGET - NPY_HEADER_MAX * len(outs)) // len(outs)
+    for name, o in zip(names, outs):
+        a = np.asarray(o.to_numpy() if isinstance(o, DeviceArray) else o)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        if a.nbytes > share:
+            flat = a.reshape(-1)
+            a = flat[np.sort(np.random.default_rng(0).integers(0, flat.size, share // flat.itemsize))]
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 def measure(spec, precision, steps, warmup, rank=0, world=1, dist=None, use_graph=True,
-            node_region=True, e2e_steps=0, seed=1234, check_truth=False):
-    """One workload on this rank's GPU.  Returns a dict of measurements (see main())."""
+            node_region=True, e2e_steps=0, seed=1234, check_truth=False, dump_dir=None):
+    """One workload on this rank's GPU.  Returns a dict of measurements (see main()).  With
+    ``dump_dir`` the outputs of the last timed step are written there (dump_outputs)."""
     import torch
 
     from aesara_b200.runtime import lib
@@ -519,12 +545,15 @@ def measure(spec, precision, steps, warmup, rank=0, world=1, dist=None, use_grap
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = None
+
     def timed_region(n):
+        nonlocal last
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         e0.record()
         for _ in range(n):
-            step()
+            last = step()
         e1.record()
         barrier()
         t = torch.tensor([e0.elapsed_time(e1)], device="cuda")
@@ -547,6 +576,10 @@ def measure(spec, precision, steps, warmup, rank=0, world=1, dist=None, use_grap
     l0 = L.ab_launch_count()
     ms_step = timed_region(steps)
     launches = L.ab_launch_count() - l0
+    if dump_dir is not None:
+        # before the next call: a replayed graph writes every step into the same output buffers
+        dump_outputs(last, spec["outputs"], dump_dir)
+    last = None
     replay = getattr(getattr(f, "vm", None), "_replay", None) or getattr(f, "replay", None)
     replayed = bool(replay is not None and replay.replays)
     res.update(ms_per_step=ms_step, executor="cuda-graph replay" if replayed else "eager launches")
@@ -771,10 +804,47 @@ def roofline_of(spec, precision, m, peaks):
             "algorithmic_bytes": nbytes}
 
 
+def private_caches():
+    """Where the tree cannot be written, point the caches the benchmark fills at run time at a
+    temporary directory: the JIT kernel cache becomes links to the cubins the build left in
+    aesara_b200/_kcache (kernels compiled now are added beside them), and the front-end's
+    C-linker compiles into an empty directory instead of oracle/_ref/compiledir.  A writable
+    tree keeps both caches in place; they are git-ignored."""
+    import atexit
+    import shutil
+    import tempfile
+
+    def writable(p):
+        while not os.path.exists(p):
+            p = os.path.dirname(p)
+        return os.access(p, os.W_OK)
+
+    kcache = os.path.join(ROOT, "aesara_b200", "_kcache")
+    compiledir = os.path.join(ROOT, "oracle", "_ref", "compiledir")
+    move_k = not os.environ.get("AESARA_B200_CACHE") and not writable(kcache)
+    move_c = (not os.environ.get("AESARA_B200_COMPILEDIR") and os.path.isdir(os.path.dirname(compiledir))
+              and not writable(compiledir))
+    if not (move_k or move_c):
+        return
+    d = tempfile.mkdtemp(prefix="aesara_b200_bench_")
+    atexit.register(shutil.rmtree, d, True)
+    if move_k:
+        kc = os.path.join(d, "kernels")
+        os.makedirs(kc)
+        if os.path.isdir(kcache):
+            for name in os.listdir(kcache):
+                if name.endswith(".cubin"):
+                    os.symlink(os.path.join(kcache, name), os.path.join(kc, name))
+        os.environ["AESARA_B200_CACHE"] = kc
+    if move_c:
+        os.environ["AESARA_B200_COMPILEDIR"] = os.path.join(d, "compiledir")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps; with --impl reference at most this many, within a 150 s budget")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="mlp", choices=["mlp", "elemwise", "lstm", "logreg", "readme"])
@@ -789,7 +859,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the one-liners of the other configs")
     ap.add_argument("--no-truth", action="store_true", help="skip the float64 parity check of the headline run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32/float64, "
+                         "64 MB in all: large outputs as a fixed sample of elements); not with --impl reference")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the device path computed; --impl reference has no such outputs")
+    private_caches()
     spec = workload_spec(args.workload, args.batch, args.hidden, args.n, args.steps_t)
     if args.precision is None:
         args.precision = "bf16" if args.workload == "mlp" else "fp32"
@@ -818,8 +896,8 @@ def main():
         if parity is not None and not parity["normwise_err"] <= 4 * parity["tolerance"]:
             raise SystemExit(f"sharded evaluation disagrees with the single-GPU one: {parity}")
     m = measure(spec, args.precision, args.steps, args.warmup, rank, world, dist,
-                use_graph=bool(args.graph), e2e_steps=0 if args.no_e2e else max(2, min(args.steps, 5)),
-                check_truth=not args.no_truth)
+                use_graph=bool(args.graph), e2e_steps=0 if args.no_e2e else args.steps,
+                check_truth=not args.no_truth, dump_dir=args.dump_outputs if rank == 0 else None)
     ms_step = m["ms_per_step"]
     value = world * 1e3 / ms_step  # every rank evaluates its shard once per step
     roofline = roofline_of(spec, args.precision, m, peaks)

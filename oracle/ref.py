@@ -74,12 +74,10 @@ def materialise(force=False, verbose=True):
 
 
 def reference_dir():
-    """Directory containing the reference ``aesara`` package: the travelling copy if it
-    exists, else the build container's /root/reference, else None."""
+    """Directory containing the reference ``aesara`` package: the copy ``materialise()`` made,
+    else None.  Tests, ``smoke()`` and the benchmark read only that copy, never the source."""
     if os.path.isdir(os.path.join(REF_DIR, "aesara")):
         return REF_DIR
-    if os.path.isdir(os.path.join(SOURCE, "aesara")):
-        return SOURCE
     return None
 
 

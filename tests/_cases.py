@@ -18,6 +18,49 @@ from aesara_b200.ir import Program
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 BLAS_OPS = {"Dot22", "Dot22Scalar", "Gemm", "Gemv", "Ger", "Dot", "Scan"}
 
+# The five BASELINE graphs at the sizes tests/test_gpu_function.py calls them with: committed
+# program, graph builder in aesara_b200.graphs, seeded inputs.  c_linker_baseline.npz holds the
+# reference C-linker's outputs for these calls (tests/golden/make_golden.py --c-linker), so that
+# the comparison also runs where the Aesara front-end is not installed.
+BASELINE_CALLS = {
+    "cfg1": ("cfg1_readme", "cfg1_readme", lambda G: G.cfg1_inputs(300)),
+    "cfg2": ("cfg2_fused", "cfg2_fused_elemwise", lambda G: G.cfg2_inputs(100003, yscale=12.0)),
+    "cfg3": ("cfg3_mlp", "cfg3_mlp", lambda G: G.cfg3_inputs(384, 256)),
+    "cfg4": ("cfg4_lstm", "cfg4_lstm_scan", lambda G: G.cfg4_inputs(6, 256, 64)),
+    "cfg5": ("cfg5_logreg", "cfg5_logreg", lambda G: G.cfg5_inputs(5000, 128)),
+}
+C_LINKER_GOLDEN = os.path.join(GOLDEN, "c_linker_baseline.npz")
+C_LINKER_SAMPLE = 8192  # outputs larger than this are stored at a fixed, seeded sample of positions
+
+
+def sample_positions(size):
+    """Flat positions stored of an output with ``size`` elements (None: all of them)."""
+    if size <= C_LINKER_SAMPLE:
+        return None
+    return np.sort(np.random.default_rng(size).choice(size, C_LINKER_SAMPLE, replace=False))
+
+
+def assert_matches_c_linker(name, got):
+    """``got`` (the outputs of BASELINE_CALLS[name]) against the stored C-linker outputs, at the
+    stored positions; ``cfg2`` is the only graph without a dot product."""
+    z = np.load(C_LINKER_GOLDEN)
+    n = sum(1 for f in z.files if f.startswith(f"{name}_out_"))
+    assert len(got) == n, f"{name}: {len(got)} outputs, {n} stored"
+    for k, g in enumerate(got):
+        g = np.asarray(g)
+        if f"{name}_pos_{k}" in z.files:
+            g = g.reshape(-1)[z[f"{name}_pos_{k}"]]
+        assert_matches(g, z[f"{name}_out_{k}"], blas=name != "cfg2", what=f"{name} output {k} vs the C-linker")
+
+
+def shardplan_mixed_graph(at):
+    """Inputs and outputs of the hand-built graph of tests/test_shardplan.py, on the front-end's
+    ``aesara.tensor`` module ``at``; lowered (``FAST_COMPILE``) it is golden/programs/
+    shardplan_mixed_outputs.json."""
+    X, w = at.fmatrix("X"), at.fvector("w")
+    z = at.tanh(X @ w)
+    return [X, w], [(z ** 2).sum(), at.dot(X.T, z), z * 2, w * 3, (X ** 2).sum(axis=0) / X.shape[0]]
+
 
 def case_names():
     return sorted(os.path.basename(p)[:-5] for p in glob.glob(os.path.join(GOLDEN, "*.json")))

@@ -877,5 +877,44 @@ def main(names):
         print(f"{name}: {len(prog.nodes)} nodes {prog.op_counts()}")
 
 
+def c_linker_baseline():
+    """The reference C-linker's outputs of the BASELINE calls of tests/_cases.py (sampled where
+    large) -> c_linker_baseline.npz."""
+    from aesara.compile.mode import Mode
+
+    from tests._cases import BASELINE_CALLS, C_LINKER_GOLDEN, sample_positions
+
+    blob = {}
+    for name, (_, graph, inputs) in BASELINE_CALLS.items():
+        i, o = getattr(G, graph)()
+        f = aesara.function(i, o, mode=Mode("cvm", "fast_run"), on_unused_input="ignore")
+        for k, v in enumerate(f(*inputs(G))):
+            v = np.asarray(v)
+            pos = sample_positions(v.size)
+            if pos is None:
+                blob[f"{name}_out_{k}"] = v
+            else:
+                blob[f"{name}_pos_{k}"] = pos
+                blob[f"{name}_out_{k}"] = v.reshape(-1)[pos]
+        print(f"{name}: {len(o)} outputs")
+    np.savez_compressed(C_LINKER_GOLDEN, **blob)
+
+
+def shardplan_mixed_program():
+    """The hand-built graph of tests/test_shardplan.py::test_sum_outputs_and_mixed_graph as the
+    front-end lowers it -> programs/shardplan_mixed_outputs.json."""
+    from aesara_b200.lower import lower_fgraph
+    from tests._cases import shardplan_mixed_graph
+
+    f = aesara.function(*shardplan_mixed_graph(at), mode="FAST_COMPILE")
+    os.makedirs(os.path.join(HERE, "programs"), exist_ok=True)
+    lower_fgraph(f.maker.fgraph).save(os.path.join(HERE, "programs", "shardplan_mixed_outputs.json"))
+
+
 if __name__ == "__main__":
-    main(sys.argv[1:] or list(CASES))
+    if sys.argv[1:] == ["--c-linker"]:
+        c_linker_baseline()
+    elif sys.argv[1:] == ["--shardplan-program"]:
+        shardplan_mixed_program()
+    else:
+        main(sys.argv[1:] or list(CASES))

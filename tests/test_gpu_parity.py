@@ -63,6 +63,27 @@ def test_device_resident_call(rt, name):
         assert_matches(np.asarray(g), w, blas=uses_blas(prog), what=f"{name} out {k}")
 
 
+@pytest.mark.parametrize("name", ["cfg1", "cfg2", "cfg3", "cfg4", "cfg5"])
+def test_baseline_calls_match_the_c_linker(rt, name):
+    """The five BASELINE graphs as the linker lowers them (the committed programs), at the
+    sizes and on the seeded inputs of tests/test_gpu_function.py, against the outputs the
+    reference C-linker computed for the same calls (stored, sampled where large)."""
+    from aesara_b200 import graphs as G
+    from aesara_b200.runtime import lib
+    from tests._cases import BASELINE_CALLS, assert_matches_c_linker
+
+    program, _, inputs = BASELINE_CALLS[name]
+    prog, _, _ = load_case(program)
+    ex = rt(prog)
+    before = lib.load().ab_launch_count()
+    got = ex(*[np.array(a) for a in inputs(G)])
+    assert lib.load().ab_launch_count() > before, "no kernel of libaesara_b200.so ran"
+    assert_matches_c_linker(name, got)
+    if name == "cfg4":
+        scan = [st["runner"] for st in ex._state if "runner" in st][0]
+        assert scan.used_fast_path, "the persistent Scan kernel did not run"
+
+
 def test_host_api_pinned_uploads_overlap_and_results_are_not_recycled(rt):
     """Page-locked arguments go through the asynchronous copy stream, pageable ones
     through the synchronous path; both give the same bits.  Large outputs come back in

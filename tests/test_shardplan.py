@@ -5,6 +5,8 @@ this axis, and the outputs combine as sum / mean / concat" — is checked NUMERI
 evaluates the program on three unequal row blocks, the results are combined exactly as the plan
 says, and must equal the oracle's evaluation of the whole batch.  Graphs that are not batch maps
 must be refused with ReplicasOnly."""
+import os
+
 import numpy as np
 import pytest
 
@@ -87,25 +89,30 @@ def test_scan_batch_axis():
 
 
 def test_sum_outputs_and_mixed_graph():
-    """A hand-built program through the front-end when it is available: unnormalised sums
-    combine as `sum`, per-row values as `concat`, and parameters as `rep`."""
+    """A hand-built program, ``z = tanh(X @ w)`` -> ``[(z ** 2).sum(), X.T @ z, z * 2, w * 3,
+    (X ** 2).sum(axis=0) / X.shape[0]]`` as the front-end lowers it (``FAST_COMPILE``, stored by
+    tests/golden/make_golden.py --shardplan-program): unnormalised sums combine as `sum`, per-row
+    values as `concat`, and parameters as `rep`.  Where a front-end is available, the program it
+    lowers now is checked too."""
     from aesara_b200.compat import bootstrap
+    from aesara_b200.ir import Program
+    from tests._cases import GOLDEN, shardplan_mixed_graph
 
-    if not bootstrap.available():
-        pytest.skip("reference front-end not available")
-    aesara = bootstrap.load_aesara()
-    import aesara.tensor as at
-
-    from aesara_b200.lower import lower_fgraph
-
-    X, w = at.fmatrix("X"), at.fvector("w")
-    z = at.tanh(X @ w)
-    outs = [(z ** 2).sum(), at.dot(X.T, z), z * 2, w * 3, (X ** 2).sum(axis=0) / X.shape[0]]
-    f = aesara.function([X, w], outs, mode="FAST_COMPILE")
-    prog = lower_fgraph(f.maker.fgraph)
+    prog = Program.load(os.path.join(GOLDEN, "programs", "shardplan_mixed_outputs.json"))
     plan = S.infer_sharded_inputs(prog)
     assert plan.sharded_inputs == [0, None]
     assert [m[0] for m in plan.outputs] == ["sum", "sum", "concat", "rep", "mean"]
+    if bootstrap.available():
+        aesara = bootstrap.load_aesara()
+        import aesara.tensor as at
+
+        from aesara_b200.lower import lower_fgraph
+
+        f = aesara.function(*shardplan_mixed_graph(at), mode="FAST_COMPILE")
+        live = lower_fgraph(f.maker.fgraph)
+        assert [n.op for n in live.nodes] == [n.op for n in prog.nodes]
+        live_plan = S.infer_sharded_inputs(live)
+        assert live_plan.sharded_inputs == plan.sharded_inputs and live_plan.outputs == plan.outputs
     rng = np.random.default_rng(0)
     _check_numerically(prog, [rng.standard_normal((50, 7)).astype("float32"),
                               rng.standard_normal(7).astype("float32")], plan)
