@@ -76,19 +76,37 @@ def merge_exprs(steps, n_operands, outputs, name="region"):
             "outputs": outs, "stmts": stmts, "name": name}
 
 
+_UNIFORM_DIV = """\
+// x / d for a d that is the same for every element of the launch (codegen/scalar_cuda.py
+// emit_body).  r = ab_uniform_rcp(d) is 1 / d when d = +-2^k and 2^-k is a normal float, else
+// 0.  For such a d, x * r is the same correctly rounded value as x / d for every x (subnormal
+// results, zeros, infinities, NaN).  `fast` is a compile-time constant at every call: the
+// kernel checks r != 0 once and runs the chunk loop built for that case.
+__device__ __forceinline__ float ab_uniform_rcp(float d) {
+  const unsigned e = (__float_as_uint(d) >> 23) & 0xffu;
+  return ((__float_as_uint(d) & 0x7fffffu) == 0u && e >= 1u && e <= 253u) ? 1.0f / d : 0.0f;
+}
+__device__ __forceinline__ float ab_div_uniform(float x, float d, float r, bool fast) {
+  return fast ? x * r : x / d;
+}"""
+
+
 def gemm_region_source(merged, n_operands, colsum=-1, fullsum=-1, cin=True, pre_op=-1, tplane=-1,
-                       exact_sums=True, row_mask=0):
+                       exact_sums=True, row_mask=0, scalar_mask=0):
     """``merged``: expression from :func:`merge_exprs` (input 0 = the accumulator value).
     ``colsum`` / ``fullsum``: index of the value whose column sums / total the epilogue
     accumulates in float64 (-1: none).  ``cin``: the product has a beta*C term read from memory
     (a ``Gemm``) — read a chunk ahead; ``pre_op``: the memory operand that is a full [M, N]
-    matrix, read a chunk ahead as well (-1: none).  ``tplane``: index of the value that can
-    also be written as a transposed bf16 operand plane (-1: none; must equal ``colsum`` when
-    both are given -- the kernel keeps one value per chunk in registers for both).
+    matrix with unit column stride (the launch checks it), read a chunk ahead as well (-1:
+    none).  ``tplane``: index of the value that can also be written as a transposed bf16
+    operand plane (-1: none; must equal ``colsum`` when both are given -- the kernel keeps one
+    value per chunk in registers for both).
     ``exact_sums``: the sums inside a warp are kept as float pairs (float64-equivalent, the
     fp32-faithful policy); otherwise 8 / 32 addends at a time are added as a float32 tree (the
     tf32 / bf16 policies, whose addends carry a larger error than that already).
-    ``row_mask``: bit k set = memory operand k is statically a [1, N] row (a bias)."""
+    ``row_mask``: bit k set = memory operand k is statically a [1, N] row (a bias).
+    ``scalar_mask``: bit k set = memory operand k is statically [1, 1]: read once per kernel,
+    and a division by it is decided once per kernel (``ab_div_uniform``)."""
     if tplane >= 0 and colsum >= 0 and tplane != colsum:
         raise NotImplementedError("fused epilogue: transposed plane and column sums of different values")
     n_out = len(merged["out_dtypes"])
@@ -96,7 +114,11 @@ def gemm_region_source(merged, n_operands, colsum=-1, fullsum=-1, cin=True, pre_
         raise NotImplementedError("fused epilogue: 1..3 values")
     if n_operands > MAX_OPERANDS:
         raise NotImplementedError("fused epilogue: at most 4 memory operands")
+    scalars = [k for k in range(n_operands) if (scalar_mask >> k) & 1]
     args = ["(V)"] + [f"(E)[{k}][(T)]" for k in range(n_operands)] + [f"(O)[{k}][(T)]" for k in range(n_out)]
+    body = emit_body(merged, fn_name="ab_ep_body", uniform_divisors=[1 + k for k in scalars])
+    udiv = "ab_div_uniform(" in body
+    args += [f"(R)[{k}]" for k in scalars] + (["(F)"] if scalars else [])
     gen = [
         "// generated by aesara_b200.codegen.gemm_epilogue — " + merged.get("name", ""),
         "#define AB_EPILOGUE 1",
@@ -109,11 +131,14 @@ def gemm_region_source(merged, n_operands, colsum=-1, fullsum=-1, cin=True, pre_
         f"#define AB_EP_TPLANE ({tplane})",
         f"#define AB_EP_EXACT_SUMS {1 if exact_sums else 0}",
         f"#define AB_EP_ROWMASK {int(row_mask)}",
+        f"#define AB_EP_SCALARMASK {int(scalar_mask)}",
+        f"#define AB_EP_UDIV {1 if udiv else 0}",  # the program divides by a [1, 1] operand
         # the stored / reduced / transposed value leaves through shared memory (coalesced
         # stores, shuffle-free transposes); AB_EP_NO_STAGING=1 keeps the register-only epilogue
         f"#define AB_EP_STAGED {0 if os.environ.get('AB_EP_NO_STAGING') else 1}",
-        emit_body(merged, fn_name="ab_ep_body"),
-        "#define AB_EP_EVAL(V, E, T, O) ab_ep_body(" + ", ".join(args) + ")",
+        _UNIFORM_DIV,
+        body,
+        "#define AB_EP_EVAL(V, E, T, O, R, F) ab_ep_body(" + ", ".join(args) + ")",
         "namespace ab { namespace tc {} }",
     ]
     return "\n".join([

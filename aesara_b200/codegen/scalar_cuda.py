@@ -261,12 +261,22 @@ TABLE = {
 }
 
 
-def emit_body(expr, fn_name="ab_body"):
-    """Return CUDA source of ``__device__ void ab_body(in..., out&...)``."""
+def emit_body(expr, fn_name="ab_body", uniform_divisors=()):
+    """Return CUDA source of ``__device__ void ab_body(in..., out&...)``.
+
+    ``uniform_divisors``: indices k of float32 inputs that hold the same value for every element
+    of a launch.  The function then takes one more parameter ``r<k>`` per such input, ``1/i<k>``
+    when that is an exact power of two with a normal reciprocal, and a last ``bool udiv``: true
+    when the caller has checked, once, that every ``r<k>`` is such a reciprocal.  A float32
+    division by ``i<k>`` becomes ``ab_div_uniform(x, i<k>, r<k>, udiv)``: ``x * r<k>`` under
+    ``udiv`` (the same bits as the IEEE division, without its per-element refinement and
+    slow-path branch), the IEEE division otherwise."""
     in_dts = expr["inputs"]
     out_dts = expr["out_dtypes"]
     params = [f"const {ctype(dt)} i{k}" for k, dt in enumerate(in_dts)]
     params += [f"{ctype(dt)}& o{k}" for k, dt in enumerate(out_dts)]
+    udiv = {f"i{k}": f"r{k}" for k in uniform_divisors if in_dts[k] == "float32"}
+    params += [f"const float {r}" for r in udiv.values()] + (["const bool udiv"] if udiv else [])
     lines = [f"__device__ __forceinline__ void {fn_name}({', '.join(params)}) {{"]
 
     def ref(r):
@@ -284,7 +294,11 @@ def emit_body(expr, fn_name="ab_body"):
             raise UnsupportedScalar("statement without in_dtypes")
         for dt in list(idt) + [st["dtype"]]:
             _kind(dt)
-        rhs = gen(args, idt, st["dtype"], st)
+        if (st["op"] == "true_divide" and st["dtype"] == "float32" and list(idt) == ["float32", "float32"]
+                and args[1] in udiv):
+            rhs = f"ab_div_uniform({args[0]}, {args[1]}, {udiv[args[1]]}, udiv)"
+        else:
+            rhs = gen(args, idt, st["dtype"], st)
         lines.append(f"  const {ctype(st['dtype'])} t{k} = {rhs};")
     for k, r in enumerate(expr["outputs"]):
         lines.append(f"  o{k} = {ref(r)};")

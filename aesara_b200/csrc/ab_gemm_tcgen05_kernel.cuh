@@ -304,7 +304,10 @@ struct EpilogueOut {
   // columns of a thread (tanh, IEEE division, float64 sums per element) is several hundred KB
   // of SASS, which every warp re-fetches from L2 for every tile (measured: the region with
   // two values and two reductions ran 1.5 ms slower than its five separate kernels).
-  struct FusedScalars { float v[4]; bool is[4]; bool vec[4]; };
+  // v: the [1, 1] operands' values; rcp: ab_uniform_rcp of the statically [1, 1] ones, udiv:
+  // all of those are exact reciprocals, so the divisions by them may multiply (AB_EP_UDIV
+  // builds; codegen/gemm_epilogue.py)
+  struct FusedScalars { float v[4]; float rcp[4]; bool is[4]; bool vec[4]; bool udiv; };
   // Sums of the region are kept as unevaluated float pairs (hi + lo, error-free TwoSum) while
   // they stay inside a thread or a warp, and become float64 where they leave it: the FP64
   // pipe of this part retires a warp-wide DADD every ~20 cycles, and one DADD + one F2F.F64
@@ -331,11 +334,14 @@ struct EpilogueOut {
   }
   __device__ __forceinline__ FusedScalars load_scalars() const {
     FusedScalars s;
+    s.udiv = true;
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-      s.is[k] = k < AB_EP_NOPS && p.ep_rs[k] == 0 && p.ep_cs[k] == 0;  // a [1,1] operand
+      s.is[k] = k < AB_EP_NOPS && (is_scalar_op(k) || (p.ep_rs[k] == 0 && p.ep_cs[k] == 0));  // a [1,1] operand
       s.v[k] = s.is[k] ? p.ep_ptr[k][0] : 0.0f;
-      s.vec[k] = k < AB_EP_NOPS && p.ep_rs[k] == 0 && p.ep_cs[k] == 1;  // a [1,N] row (a bias)
+      s.rcp[k] = is_scalar_op(k) ? ab_uniform_rcp(s.v[k]) : 0.0f;
+      if (is_scalar_op(k) && s.rcp[k] == 0.0f) s.udiv = false;
+      s.vec[k] = k < AB_EP_NOPS && (is_row_op(k) || (!is_scalar_op(k) && p.ep_rs[k] == 0 && p.ep_cs[k] == 1));  // a [1,N] row (a bias)
     }
     return s;
   }
@@ -383,12 +389,16 @@ struct EpilogueOut {
 #ifndef AB_EP_ROWMASK
 #define AB_EP_ROWMASK 0
 #endif
+#ifndef AB_EP_SCALARMASK
+#define AB_EP_SCALARMASK 0
+#endif
   static __device__ __forceinline__ constexpr int popc4(unsigned m) {  // NVRTC has no __builtin_popcount
     return (int)((m & 1u) + ((m >> 1) & 1u) + ((m >> 2) & 1u) + ((m >> 3) & 1u));
   }
   static constexpr int kRowOps = ((AB_EP_ROWMASK) & 1) + (((AB_EP_ROWMASK) >> 1) & 1) +
                                  (((AB_EP_ROWMASK) >> 2) & 1) + (((AB_EP_ROWMASK) >> 3) & 1);
   static __device__ __forceinline__ constexpr bool is_row_op(int k) { return ((AB_EP_ROWMASK >> k) & 1) != 0; }
+  static __device__ __forceinline__ constexpr bool is_scalar_op(int k) { return ((AB_EP_SCALARMASK >> k) & 1) != 0; }
   static __device__ __forceinline__ constexpr int row_slot(int k) {
     return popc4((unsigned)AB_EP_ROWMASK & ((1u << k) - 1u));
   }
@@ -416,23 +426,25 @@ struct EpilogueOut {
     float vec[AB_EP_NOPS > 0 ? AB_EP_NOPS : 1];
     float rowv[kRowOps > 0 ? kRowOps : 1][32];
   };
+  // EDGE = false: the warp's 32 rows and the tile's columns are all inside [M, N] (no tests)
+  template <bool EDGE = true>
   __device__ __forceinline__ void prefetch_chunk(ChunkPre& pre, long long row, long long col0, bool live,
                                                  const FusedScalars& sc, int lane) const {
     const long long r = live ? row : 0;
     (void)r; (void)sc; (void)pre; (void)col0;
 #pragma unroll
     for (int k = 0; k < AB_EP_NOPS; ++k) {
-      if (is_row_op(k) && sc.vec[k]) {
+      if (is_row_op(k)) {
 #pragma unroll
         for (int j = 0; j < 32; j += 4) {
           // N % 8 == 0 and 16-byte aligned rows (the fused launch's contract)
-          const float4 q = (col0 + j < p.N) ? __ldg(reinterpret_cast<const float4*>(p.ep_ptr[k] + col0 + j))
-                                            : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+          const float4 q = (!EDGE || col0 + j < p.N) ? __ldg(reinterpret_cast<const float4*>(p.ep_ptr[k] + col0 + j))
+                                                     : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
           float* d = &pre.rowv[row_slot(k)][j];
           d[0] = q.x; d[1] = q.y; d[2] = q.z; d[3] = q.w;
         }
       } else if (sc.vec[k]) {
-        pre.vec[k] = (col0 + lane < p.N) ? __ldg(p.ep_ptr[k] + col0 + lane) : 0.0f;
+        pre.vec[k] = (!EDGE || col0 + lane < p.N) ? __ldg(p.ep_ptr[k] + col0 + lane) : 0.0f;
       }
     }
 #if AB_EP_STAGED
@@ -444,19 +456,20 @@ struct EpilogueOut {
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const long long grow = row0 + 4 * i + (lane >> 3);
-          pre.cinq[i] = (grow < p.M && col < p.N) ? __ldcs(reinterpret_cast<const float4*>(p.Cin + grow * p.cin_rs + col))
-                                                  : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+          pre.cinq[i] = (!EDGE || (grow < p.M && col < p.N)) ? __ldcs(reinterpret_cast<const float4*>(p.Cin + grow * p.cin_rs + col))
+                                                             : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
         }
       }
 #endif
 #if AB_EP_PRE_OP >= 0
-      if (!sc.is[AB_EP_PRE_OP] && p.ep_cs[AB_EP_PRE_OP] == 1) {
+      {
+        // a unit-stride [M, N] matrix (the launch checks it, GemmEpilogueFusion._operands_fit)
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const long long grow = row0 + 4 * i + (lane >> 3);
-          pre.opq[i] = (grow < p.M && col < p.N)
+          pre.opq[i] = (!EDGE || (grow < p.M && col < p.N))
                            ? __ldcs(reinterpret_cast<const float4*>(p.ep_ptr[AB_EP_PRE_OP] + grow * p.ep_rs[AB_EP_PRE_OP] + col))
-                           : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                                                            : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
         }
       }
 #endif
@@ -470,7 +483,7 @@ struct EpilogueOut {
     }
 #endif
 #if AB_EP_PRE_OP >= 0
-    if (live && !sc.is[AB_EP_PRE_OP] && p.ep_cs[AB_EP_PRE_OP] == 1) {
+    if (live) {
       const bool wide = ((reinterpret_cast<uintptr_t>(p.ep_ptr[AB_EP_PRE_OP]) & 31) == 0) && ((p.ep_rs[AB_EP_PRE_OP] & 7) == 0);
 #pragma unroll
       for (int j = 0; j < 32; j += 8)
@@ -481,19 +494,32 @@ struct EpilogueOut {
 #endif
   }
 #if AB_EP_STAGED
-  // coalesced layout (ChunkPre) -> this lane's row, through the staging buffer
-  __device__ __forceinline__ void restage(const float4 (&q)[8], float (&out)[32], int lane) const {
+  // coalesced layout (ChunkPre) -> the staging buffer, rows of the warp's 32 as in the tile
+  __device__ __forceinline__ void stage_in(const float4 (&q)[8], int lane) const {
 #pragma unroll
     for (int i = 0; i < 8; ++i) sts128(stage + 4u * st_off(4 * i + (lane >> 3), lane & 7), q[i].x, q[i].y, q[i].z, q[i].w);
     __syncwarp();
+  }
+  // columns j .. j + 7 of this lane's row
+  __device__ __forceinline__ void stage_group(int j, float (&out)[8], int lane) const {
+    const float4 a = lds128(stage + 4u * st_off(lane, j >> 2)), b = lds128(stage + 4u * st_off(lane, (j >> 2) + 1));
+    out[0] = a.x; out[1] = a.y; out[2] = a.z; out[3] = a.w; out[4] = b.x; out[5] = b.y; out[6] = b.z; out[7] = b.w;
+  }
+  // coalesced layout (ChunkPre) -> this lane's row, through the staging buffer
+  __device__ __forceinline__ void restage(const float4 (&q)[8], float (&out)[32], int lane) const {
+    stage_in(q, lane);
 #pragma unroll
-    for (int g = 0; g < 8; ++g) {
-      const float4 v = lds128(stage + 4u * st_off(lane, g));
-      out[4 * g] = v.x; out[4 * g + 1] = v.y; out[4 * g + 2] = v.z; out[4 * g + 3] = v.w;
-    }
+    for (int g = 0; g < 8; g += 2) stage_group(4 * g, *reinterpret_cast<float(*)[8]>(&out[4 * g]), lane);
     __syncwarp();
   }
 #endif
+  // AB_EP_LAZY: the region reads ONE [M, N] operand (Cin or the read-ahead matrix).  It stays in
+  // the staging buffer and each group of 8 columns reads its values right before their use, from
+  // this lane's own row -- the slots the group's value is staged to next, which no other lane
+  // touches before fused_reduce's __syncwarp.  Read into 32 registers at the top of the chunk
+  // instead, they are spilled in the region with Y, b2 and the loss (1.5 KB of local traffic
+  // per chunk and warp).
+#define AB_EP_LAZY (AB_EP_STAGED && (AB_EP_CIN + (AB_EP_PRE_OP >= 0 ? 1 : 0)) == 1)
   // ---- one 32-column chunk of one accumulator row, in two parts -------------------------
   // fused_eval:   x[32] (raw accumulator values of columns col0 .. col0+31 of `row`) -> the
   //               region's values; consumes the read-ahead buffer `pre`, stores the outputs and
@@ -506,21 +532,26 @@ struct EpilogueOut {
   // (Two alternating buffers and a loop body of two chunks did the same at twice the code:
   // ~4900 SASS instructions per iteration, 35 % of the epilogue warps' samples waiting for
   // instruction fetch -- stall_no_inst, profiles/r02_region2_tplane_icache.txt.)
+  // UDIV: multiply by the reciprocals of the [1, 1] divisors (FusedScalars::udiv holds)
+  template <bool EDGE = true, bool UDIV = false>
   __device__ __forceinline__ void fused_eval(float (&x)[32], long long row, long long col0, bool live,
                                              int lane, const FusedScalars& sc, FF& fs, const ChunkPre& pre) const {
     const long long r = live ? row : 0;
     (void)lane; (void)fs;
-#if AB_EP_PRE_OP >= 0
-    const bool pre_ok = live && !sc.is[AB_EP_PRE_OP] && p.ep_cs[AB_EP_PRE_OP] == 1;
+#if AB_EP_LAZY
+#if AB_EP_CIN
+    if (p.beta != 0.0f) stage_in(pre.cinq, lane);
+#else
+    stage_in(pre.opq, lane);
 #endif
-#if AB_EP_STAGED
+#elif AB_EP_STAGED
 #if AB_EP_CIN
     float cin_l[32];
     if (p.beta != 0.0f) restage(pre.cinq, cin_l, lane);
 #endif
 #if AB_EP_PRE_OP >= 0
     float op_l[32];
-    if (!sc.is[AB_EP_PRE_OP] && p.ep_cs[AB_EP_PRE_OP] == 1) restage(pre.opq, op_l, lane);
+    restage(pre.opq, op_l, lane);
 #endif
 #else
 #if AB_EP_CIN
@@ -537,7 +568,7 @@ struct EpilogueOut {
       float ev[AB_EP_NOPS > 0 ? AB_EP_NOPS : 1][8];
 #pragma unroll
       for (int k = 0; k < AB_EP_NOPS; ++k) {
-        if (is_row_op(k) && sc.vec[k]) {
+        if (is_row_op(k)) {
 #pragma unroll
           for (int t = 0; t < 8; ++t) ev[k][t] = pre.rowv[row_slot(k)][j + t];
         } else if (sc.vec[k]) {
@@ -545,14 +576,21 @@ struct EpilogueOut {
           for (int t = 0; t < 8; ++t) ev[k][t] = __shfl_sync(0xffffffffu, pre.vec[k], j + t);
         }
       }
-      if (live && col < p.N) {  // N % 8 == 0: a group of 8 columns is inside or outside as a whole
+      if (!EDGE || (live && col < p.N)) {  // N % 8 == 0: a group of 8 columns is inside or outside as a whole
         float v[8];
 #pragma unroll
         for (int t = 0; t < 8; ++t) v[t] = p.alpha * x[j + t];
         if (p.beta != 0.0f) {
 #if AB_EP_CIN
+#if AB_EP_LAZY
+          float cin_g[8];
+          stage_group(j, cin_g, lane);
+#pragma unroll
+          for (int t = 0; t < 8; ++t) v[t] += p.beta * cin_g[t];
+#else
 #pragma unroll
           for (int t = 0; t < 8; ++t) v[t] += p.beta * cin_l[j + t];
+#endif
 #else
           float ci[8];
           ld8<true>(p.Cin + r * p.cin_rs + col, ci, wide_in);
@@ -564,13 +602,17 @@ struct EpilogueOut {
 #pragma unroll
         for (int k = 0; k < AB_EP_NOPS; ++k) {
 #if AB_EP_PRE_OP >= 0
-          if (k == AB_EP_PRE_OP && pre_ok) {
+          if (k == AB_EP_PRE_OP) {
+#if AB_EP_LAZY
+            stage_group(j, e[k], lane);
+#else
 #pragma unroll
             for (int t = 0; t < 8; ++t) e[k][t] = op_l[j + t];
+#endif
             continue;
           }
 #endif
-          if (sc.vec[k]) {
+          if (is_row_op(k) || sc.vec[k]) {
 #pragma unroll
             for (int t = 0; t < 8; ++t) e[k][t] = ev[k][t];
           } else if (sc.is[k]) {
@@ -587,7 +629,7 @@ struct EpilogueOut {
         }
         float o[AB_EP_NOUT][8];
 #pragma unroll
-        for (int t = 0; t < 8; ++t) { AB_EP_EVAL(v[t], e, t, o); }
+        for (int t = 0; t < 8; ++t) { AB_EP_EVAL(v[t], e, t, o, sc.rcp, UDIV); }
 #if AB_EP_STAGED
         put_outputs<kStageValue>(o, r, col);
         sts128(stage + 4u * st_off(lane, j >> 2), o[kStageValue][0], o[kStageValue][1], o[kStageValue][2], o[kStageValue][3]);
@@ -657,6 +699,7 @@ struct EpilogueOut {
   static constexpr int kStageValue = AB_EP_COLSUM >= 0 ? AB_EP_COLSUM : (AB_EP_TPLANE >= 0 ? AB_EP_TPLANE : 0);
   static __device__ __forceinline__ uint32_t st_off(int r, int g) { return (uint32_t)(r * 32 + ((g ^ (r & 7)) << 2)); }
 #if AB_EP_STAGED
+  template <bool EDGE = true>
   __device__ __forceinline__ void fused_reduce(float (&x)[32], long long row, long long col0, int lane) const {
     (void)x;
     __syncwarp();
@@ -673,7 +716,7 @@ struct EpilogueOut {
           const int r = 4 * i + (lane >> 3);
           const float4 v = lds128(stage + 4u * st_off(r, g));
           const long long grow = row0 + r;
-          if (grow < p.M && col < p.N) {
+          if (!EDGE || (grow < p.M && col < p.N)) {
             if (dst != nullptr) __stcs(reinterpret_cast<float4*>(dst + grow * rs + col), v);
             if (sp != nullptr) {
               uint32_t h0, h1;
@@ -733,13 +776,13 @@ struct EpilogueOut {
           }
           const double tot = (double)t16[0];
 #endif
-          if (rb * 32 < p.M && c < p.N) p.colsum_ws[rb * p.N + c] = tot;
+          if (!EDGE || (rb * 32 < p.M && c < p.N)) p.colsum_ws[rb * p.N + c] = tot;
         }
 #endif
 #if AB_EP_TPLANE >= 0
-        if (want_t && c < p.N && row0 < p.M) {
+        if (want_t && (!EDGE || (c < p.N && row0 < p.M))) {
           uint16_t* dst = static_cast<uint16_t*>(p.shadow_t) + c * p.shadow_t_pitch + row0;
-          if (row0 + 32 <= p.M) {
+          if (!EDGE || row0 + 32 <= p.M) {
             uint32_t h[16];
 #pragma unroll
             for (int t = 0; t < 16; ++t)
@@ -764,6 +807,7 @@ struct EpilogueOut {
     __syncwarp();  // the buffer is free for the next chunk's values
   }
 #else
+  template <bool EDGE = true>
   __device__ __forceinline__ void fused_reduce(float (&x)[32], long long row, long long col0, int lane) const {
     (void)x; (void)row; (void)col0; (void)lane;
 #if AB_EP_TPLANE >= 0
@@ -909,12 +953,17 @@ struct EpilogueOut {
   // the whole K range sits in one TMEM accumulator (bf16 / tf32 policies): 32 columns at a
   // time straight from TMEM in a rolled loop -- 32 live accumulator registers instead of 128,
   // and the body exists once
-  __device__ __forceinline__ void store_fused_tmem(uint32_t t_acc, long long row, long long n0, int nchunks,
-                                                   int lane, const FusedScalars& sc) const {
-    const bool live = row < p.M;
-    FF fs = {0.0f, 0.0f};
+  //
+  // A tile whose rows (this warp's 32) and columns all lie inside [M, N] -- every tile of a
+  // problem whose sizes are multiples of the tile -- runs the chunk loop without any row or
+  // column test (EDGE = false); only the tiles on the bottom / right border take the checked
+  // loop.  The two loops are separate bodies: a tile never runs instructions of both.
+  template <bool EDGE, bool UDIV>
+  __device__ __forceinline__ void chunk_loop(uint32_t t_acc, long long row, long long n0, int nchunks,
+                                             int lane, const FusedScalars& sc, FF& fs) const {
+    const bool live = !EDGE || row < p.M;
     ChunkPre pre;
-    prefetch_chunk(pre, row, n0, live, sc, lane);
+    prefetch_chunk<EDGE>(pre, row, n0, live, sc, lane);
 #pragma unroll 1
     for (int c = 0; c < nchunks; ++c) {
       uint32_t r[32];
@@ -923,10 +972,24 @@ struct EpilogueOut {
 #pragma unroll
       for (int j = 0; j < 32; ++j) x[j] = __uint_as_float(r[j]);
       const long long col0 = n0 + c * 32;
-      fused_eval(x, row, col0, live, lane, sc, fs, pre);
-      if (c + 1 < nchunks) prefetch_chunk(pre, row, col0 + 32, live, sc, lane);
-      fused_reduce(x, row, col0, lane);
+      fused_eval<EDGE, UDIV>(x, row, col0, live, lane, sc, fs, pre);
+      if (c + 1 < nchunks) prefetch_chunk<EDGE>(pre, row, col0 + 32, live, sc, lane);
+      fused_reduce<EDGE>(x, row, col0, lane);
     }
+  }
+  __device__ __forceinline__ void store_fused_tmem(uint32_t t_acc, long long row, long long n0, int nchunks,
+                                                   int lane, const FusedScalars& sc) const {
+    FF fs = {0.0f, 0.0f};
+    const bool interior = row - lane + 32 <= p.M && n0 + 32 * nchunks <= p.N;  // warp-uniform
+#if AB_EP_UDIV
+    if (interior && sc.udiv)
+      chunk_loop<false, true>(t_acc, row, n0, nchunks, lane, sc, fs);
+    else
+#endif
+    if (interior)
+      chunk_loop<false, false>(t_acc, row, n0, nchunks, lane, sc, fs);
+    else
+      chunk_loop<true, false>(t_acc, row, n0, nchunks, lane, sc, fs);
     finish_fullsum(fs, row, n0, lane);
   }
 #endif  // AB_EPILOGUE

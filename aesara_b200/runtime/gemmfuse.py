@@ -129,6 +129,7 @@ class GemmEpilogueFusion:
         self.broken = False
         self.f32_skipped = 0                  # values kept as a bf16 plane only (last run)
         self._src = None
+        self._pre_op = -1
         self._handle = None
 
     # ------------------------------------------------------------------ analysis
@@ -331,17 +332,34 @@ class GemmEpilogueFusion:
                 if c is None and not (ss is not None and len(ss) == 2 and ss[0] == 1):
                     pre_op = k
                     break
-            # operands that are statically [1, N] rows with N unknown or > 1 (biases)
-            row_mask = 0
-            for k, v in enumerate(self.operand_vars):
-                ss = prog.vars[v].static_shape
-                if ss is not None and len(ss) == 2 and ss[0] == 1 and ss[1] != 1:
-                    row_mask |= 1 << k
             self._src = gemm_region_source(merged, len(self.operand_vars), self.colsum, self.fullsum,
                                            cin=prog.nodes[self.g].op == "Gemm", pre_op=pre_op,
                                            tplane=self.tplane if self.planes else -1,
-                                           exact_sums=self.exact_sums, row_mask=row_mask)
+                                           exact_sums=self.exact_sums, row_mask=self._kind_mask("row"),
+                                           scalar_mask=self._kind_mask("scalar"))
+            self._pre_op = pre_op
         return self._src
+
+    def _kind_mask(self, kind):
+        """Operands whose shape is known statically: ``row`` = [1, N] with N unknown or > 1 (a
+        bias), ``scalar`` = [1, 1]."""
+        mask = 0
+        for k, v in enumerate(self.operand_vars):
+            ss = self.program.vars[v].static_shape
+            if ss is not None and len(ss) == 2 and ss[0] == 1 and (ss[1] == 1) == (kind == "scalar"):
+                mask |= 1 << k
+        return mask
+
+    def _operands_fit(self, ops, M, N):
+        """The module was generated for these operand shapes: the read-ahead matrix is [M, N]
+        and the row operands are [1, N], both with unit column stride."""
+        self.source()
+        rows = self._kind_mask("row")
+        for k, a in enumerate(ops):
+            want = (M, N) if k == self._pre_op else ((1, N) if (rows >> k) & 1 else None)
+            if want is not None and (a.shape != want or (N > 1 and a.strides[1] != 1)):
+                return False
+        return True
 
     def compile_all(self):
         _lib.compile_cubin(self.source(), "gemm_ep")
@@ -372,6 +390,8 @@ class GemmEpilogueFusion:
         for a in ops:
             if a.dtype != np.float32 or a.ndim != 2 or a.shape[0] not in (1, M) or a.shape[1] not in (1, N):
                 return False
+        if not self._operands_fit(ops, M, N):
+            return False
         plan = []
         for k, v in enumerate(self.out_vars):
             if v is None:
